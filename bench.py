@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- shapes/sec of LION's sampling hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch 32]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch 32] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
            --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -67,7 +67,35 @@ def parse():
     ap.add_argument("--e2e-compare", action="store_true", help="(diagnostic) also time the other --e2e-upload mode")
     ap.add_argument("--clock-period-ms", type=int, default=1000, help="nvidia-smi sampling period during the timed region")
     ap.add_argument("--allow-knobs", action="store_true", help="run although LION_* performance knobs are set (they are recorded in the line)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed passes, write what the last one returned as DIR/<name>.npy (float32; rank 0) "
+                         "so that two builds can be compared output for output")
     return ap.parse_args()
+
+
+DUMP_MAX_ELEMS = 4 << 20          # per array: 16 MB of float32, so that a dump stays below 64 MB in all
+
+
+def dump_outputs(dst, result):
+    """Write the 5-tuple returned by generate_samples_vada_2prior as float32 .npy files: the point clouds, the sampled
+    latents, their statistics, the NFE count and a fixed sample of the latent-point trajectory (pred_x, T x B x 8192
+    floats: the same 4096 positions of every step).  An array larger than DUMP_MAX_ELEMS is replaced by its values at
+    a fixed seeded set of flat positions.  The wall-clock sampling time is not an output and is not written."""
+    import numpy as np
+    import torch
+    image, nfe, time_ode_solve, _sampling_time, output = result
+    traj = output["eps_list"]["pred_x"]
+    n = traj[0].numel()
+    pos = torch.from_numpy(np.sort(np.random.RandomState(0).choice(n, min(n, 4096), replace=False))).to(traj[0].device)
+    arrays = {"image": image, "nfe": nfe, "time_ode_solve": time_ode_solve, "sampled_eps": output["sampled_eps"],
+              "sample_mean_global": output["print/sample_mean_global"], "sample_var_global": output["print/sample_var_global"],
+              "pred_x_sample": torch.stack([x.reshape(-1)[pos] for x in traj])}
+    os.makedirs(dst, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().float().cpu().numpy()
+        if a.size > DUMP_MAX_ELEMS:
+            a = a.ravel()[np.sort(np.random.RandomState(1).choice(a.size, DUMP_MAX_ELEMS, replace=False))]
+        np.save(os.path.join(dst, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -374,7 +402,8 @@ def main():
         if record:
             ev[0].record()
         torch.manual_seed(seed * 1000 + rank)             # distinct noise per rank (SURVEY.md 8e)
-        img, *_ = generate_samples_vada_2prior(shape, dae, diff, vae, B, False)
+        result = generate_samples_vada_2prior(shape, dae, diff, vae, B, False)
+        img = result[0]
         launches["n"] += L.last_launches(dev)             # decoder pass (the sampling loops count themselves)
         if record:
             ev[1].record()
@@ -386,7 +415,7 @@ def main():
         if record:
             ev[2].record()
             pass_events.append(ev)
-        return img
+        return result
 
     def drain():
         for i in (0, 1):
@@ -412,8 +441,10 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     e0.record()
+    last = None
     for i in range(args.steps):
-        img = one_pass(100 + i, record=True)
+        last = None                                       # the previous pass's 1 GB trajectory goes back to the allocator first
+        last = one_pass(100 + i, record=True)
     t_d0 = torch.cuda.Event(enable_timing=True); t_d0.record()
     drain()                                               # every gather has landed: inside the timed region
     e1.record()
@@ -426,7 +457,10 @@ def main():
     ms = tms.item()
     value = world * B * args.steps / (ms / 1000.0)
     n_launch = launches["n"] + diff.total_gpu_launches
-    assert torch.isfinite(img).all()
+    assert torch.isfinite(last[0]).all()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)             # before any later pass reuses the sampler's buffers
+    del last
     per_rank = None
     if world > 1:
         mine = torch.tensor([[ev[0].elapsed_time(ev[1]), ev[1].elapsed_time(ev[2])] for ev in pass_events] +

@@ -7,9 +7,11 @@ own (the reference's recipe is a JIT `load()` inside backend.py:8-27 that writes
 sources, which are read-only here).  No reference source is copied into this repo; only the
 built `_pvcnn_backend.so` lands in oracle/_ref/ (git-ignored, shipped to the GPU box).
 
-It is used by `tests/` (-m gpu) as the ground truth for the index-producing ops (FPS, ball
-query, 3-NN, voxel indices) -- their results depend on nvcc's FMA contraction, which a CPU
-restatement can only approximate -- and never by the product path.
+Its outputs on the GPU tests' inputs are the ground truth stored in tests/golden/ref_*.npz by
+tests/golden/make_golden_ref_kernels.py, above all for the index-producing ops (FPS, ball query,
+3-NN, voxel indices) -- their results depend on nvcc's FMA contraction, which a CPU restatement can
+only approximate.  bench.py's `parity` and `gpu_baseline` legs use it where it was built; the
+product path never does.
 
 The Chamfer extension (third_party/ChamferDistancePytorch/chamfer3D/{chamfer_cuda.cpp,
 chamfer3D.cu}, JIT-loaded by dist_chamfer_3D.py:12-16 with default flags) is built the same way

@@ -1,13 +1,15 @@
-"""The seven point/voxel operators through the C ABI, against (a) the CPU oracle and (b) the
-reference's own CUDA kernels compiled into oracle/_ref (bit-exact for every index output)."""
+"""The seven point/voxel operators through the C ABI, against (a) the CPU oracle and (b) the outputs of the
+reference's own CUDA kernels on the same inputs, stored in tests/golden/ref_point_ops.npz by
+tests/golden/make_golden_ref_kernels.py (bit-exact for every index output)."""
 import numpy as np
 import pytest
 import torch
 
 from oracle import point_ops as P
-from tests.util import assert_close, gen
+from tests.util import RefGolden, assert_close, gen
 
 pytestmark = pytest.mark.gpu
+REF = RefGolden("ref_point_ops")
 
 
 def _F():
@@ -15,24 +17,64 @@ def _F():
     return F
 
 
-def _ref():
-    """The reference's own kernels (oracle/_ref/_pvcnn_backend.so, built by __graft_entry__.build() in the
-    container and shipped with the snapshot).  Their absence is a FAILURE, not a silent oracle-vs-self pass."""
-    from oracle.build_ref import load_ref
-    ref = load_ref()
-    assert ref is not None, "oracle/_ref/_pvcnn_backend.so is missing: run `python oracle/build_ref.py` (needs /root/reference)"
-    return ref
+def key(test, *params):
+    return test + "/" + "_".join(str(p) for p in params)
 
 
 def cloud(seed, B, N, spread=0.5):
     return gen(seed, B, 3, N, scale=spread)
 
 
-@pytest.mark.parametrize("B,N,r", [(2, 2048, 32), (3, 1024, 16), (2, 256, 8), (1, 64, 8)])
+# Inputs of every case that is compared with the reference kernels; make_golden_ref_kernels.py runs the reference on
+# exactly these.
+VOXELIZE_CASES = [(2, 2048, 32), (3, 1024, 16), (2, 256, 8), (1, 64, 8)]
+DEVOX_CASES = [(2, 32, 2048, 32), (2, 64, 1024, 16), (1, 130, 64, 8)]
+FPS_CASES = [(3, 2048, 1024), (2, 1024, 256), (2, 256, 64), (4, 64, 16), (1, 700, 33)]
+BALL_QUERY_CASES = [(2, 2048, 1024, 0.1), (2, 1024, 256, 0.2), (2, 256, 64, 0.4), (2, 64, 16, 0.8)]
+THREE_NN_CASES = [(2, 192, 64, 16), (2, 192, 256, 64), (2, 64, 1024, 256), (2, 17, 2048, 1024)]
+
+
+def voxelize_inputs(B, N, r):
+    return cloud(1, B, N), gen(2, B, 7, N)
+
+
+def devox_inputs(B, C, N, r):
+    grid = gen(4, B, C, r, r, r)
+    coords = torch.rand(B, 3, N, generator=torch.Generator().manual_seed(5)) * (r - 1)
+    coords[:, :, :8] = torch.floor(coords[:, :, :8])       # exact lattice points: hi offset must be 0
+    coords[:, :, 8] = r - 1                                 # upper corner of the grid
+    coords[:, :, 9] = 0
+    return grid, coords
+
+
+def fps_inputs(B, N, M):
+    coords = cloud(6, B, N)
+    if N >= 256:
+        coords[0, :, 100:140] = coords[0, :, 7:8]          # duplicates => exact ties in the distances
+    return coords
+
+
+def ball_query_inputs(B, N, M, radius):
+    pts = cloud(7, B, N, spread=0.3)
+    ctr = pts[:, :, :M].clone()
+    ctr[0, :, 0] = 50.0                                     # a centre with no neighbour: all zeros
+    return pts, ctr
+
+
+def three_nn_inputs(B, C, N, M):
+    pts = cloud(9, B, N)
+    ctr = pts[:, :, :M].clone()                            # centres coincide with points: d = 0 -> clamp 1e-10
+    return pts, ctr, gen(10, B, C, M)
+
+
+def fused_inputs():
+    return cloud(29, 32, 2048, spread=0.41), gen(30, 32, 8, 2048)
+
+
+@pytest.mark.parametrize("B,N,r", VOXELIZE_CASES)
 def test_voxel_coords_and_avg_voxelize(B, N, r):
     F = _F()
-    coords = cloud(1, B, N)
-    feats = gen(2, B, 7, N)
+    coords, feats = voxelize_inputs(B, N, r)
     nc_cpu, _ = P.voxel_coords(coords, r)                    # torch-CPU summation order: values agree to rounding
     nc, vox = F.voxel_coords(coords.cuda(), r)
     assert_close(nc, nc_cpu, 2e-6, "norm_coords")
@@ -44,10 +86,10 @@ def test_voxel_coords_and_avg_voxelize(B, N, r):
     out = F.avg_voxelize(feats.cuda(), vox, r)
     out_o, ind_o, cnt_o = P.avg_voxelize(feats, vox.cpu(), r)
     assert_close(out, out_o, 1e-5, "avg_voxelize")
-    ref = _ref()
-    o, ind, cnt = ref.avg_voxelize_forward(feats.cuda(), vox.contiguous(), r)
-    assert torch.equal(ind.cpu(), ind_o) and torch.equal(cnt.cpu(), cnt_o)
-    assert_close(out.view(B, 7, -1), o, 1e-5, "avg_voxelize vs reference kernel")
+    k = key("voxelize", B, N, r)
+    REF.exact(k + "/ind", ind_o, "avg_voxelize indices: oracle vs reference kernel")
+    REF.exact(k + "/cnt", cnt_o, "avg_voxelize counts: oracle vs reference kernel")
+    REF.close(k + "/out", out.view(B, 7, -1), 1e-5, "avg_voxelize vs reference kernel")
 
 
 def test_avg_voxelize_collisions_and_single_point():
@@ -61,51 +103,38 @@ def test_avg_voxelize_collisions_and_single_point():
     assert_close(out, out_o, 1e-5, "avg_voxelize collisions")
 
 
-@pytest.mark.parametrize("B,C,N,r", [(2, 32, 2048, 32), (2, 64, 1024, 16), (1, 130, 64, 8)])
+@pytest.mark.parametrize("B,C,N,r", DEVOX_CASES)
 def test_trilinear_devoxelize(B, C, N, r):
     F = _F()
-    grid = gen(4, B, C, r, r, r)
-    coords = torch.rand(B, 3, N, generator=torch.Generator().manual_seed(5)) * (r - 1)
-    coords[:, :, :8] = torch.floor(coords[:, :, :8])       # exact lattice points: hi offset must be 0
-    coords[:, :, 8] = r - 1                                 # upper corner of the grid
-    coords[:, :, 9] = 0
+    grid, coords = devox_inputs(B, C, N, r)
     out = F.trilinear_devoxelize(grid.cuda(), coords.cuda(), r, False)
     assert_close(out, P.trilinear_devoxelize(grid, coords, r), 2e-6, "trilinear_devoxelize")
-    ref = _ref()
-    o, inds, wgts = ref.trilinear_devoxelize_forward(r, True, coords.cuda(), grid.view(B, C, -1).cuda())
-    assert_close(out, o, 1e-6, "devox vs reference kernel")
+    k = key("devox", B, C, N, r)
+    REF.close(k + "/out", out, 1e-6, "devox vs reference kernel")
     idx_o, w_o = P.trilinear_corners(coords, r)
-    assert torch.equal(inds.cpu().long(), idx_o)
-    assert torch.equal(wgts.cpu(), w_o)
+    REF.exact(k + "/inds", idx_o, "devox corner indices: oracle vs reference kernel")
+    REF.exact(k + "/wgts", w_o, "devox corner weights: oracle vs reference kernel")
 
 
-@pytest.mark.parametrize("B,N,M", [(3, 2048, 1024), (2, 1024, 256), (2, 256, 64), (4, 64, 16), (1, 700, 33)])
+@pytest.mark.parametrize("B,N,M", FPS_CASES)
 def test_furthest_point_sampling(B, N, M):
     from lion_b200.third_party.pvcnn.functional import furthest_point_sample_indices
     F = _F()
-    coords = cloud(6, B, N)
-    if N >= 256:
-        coords[0, :, 100:140] = coords[0, :, 7:8]          # duplicates => exact ties in the distances
+    coords = fps_inputs(B, N, M)
     idx = furthest_point_sample_indices(coords.cuda(), M)
-    ref = _ref()
-    idx_r = ref.furthest_point_sampling(coords.cuda(), M)
-    assert torch.equal(idx.cpu(), idx_r.cpu()), "FPS differs from the reference kernel"
+    REF.exact(key("fps", B, N, M) + "/idx", idx, "FPS indices")
     idx_o = P.furthest_point_sample_idx(coords, M)
     assert torch.equal(idx.cpu(), idx_o), "FPS differs from the oracle"
     centers = F.furthest_point_sample(coords.cuda(), M)
     assert torch.equal(centers.cpu(), P.gather(coords, idx_o))
 
 
-@pytest.mark.parametrize("B,N,M,radius", [(2, 2048, 1024, 0.1), (2, 1024, 256, 0.2), (2, 256, 64, 0.4), (2, 64, 16, 0.8)])
+@pytest.mark.parametrize("B,N,M,radius", BALL_QUERY_CASES)
 def test_ball_query_and_grouping(B, N, M, radius):
     F = _F()
-    pts = cloud(7, B, N, spread=0.3)
-    ctr = pts[:, :, :M].clone()
-    ctr[0, :, 0] = 50.0                                     # a centre with no neighbour: all zeros
+    pts, ctr = ball_query_inputs(B, N, M, radius)
     idx = F.ball_query(ctr.cuda(), pts.cuda(), radius, 32)
-    ref = _ref()
-    idx_r = ref.ball_query(ctr.cuda(), pts.cuda(), radius, 32)
-    assert torch.equal(idx.cpu(), idx_r.cpu()), "ball query differs from the reference kernel"
+    REF.exact(key("ball_query", B, N, M, radius) + "/idx", idx, "ball query indices")
     idx_o = P.ball_query(ctr, pts, radius, 32)
     assert torch.equal(idx.cpu(), idx_o), "ball query differs from the oracle"
     assert (idx[0, 0] == 0).all()
@@ -114,20 +143,17 @@ def test_ball_query_and_grouping(B, N, M, radius):
     assert torch.equal(g.cpu(), P.grouping(feats, idx_o))
 
 
-@pytest.mark.parametrize("B,C,N,M", [(2, 192, 64, 16), (2, 192, 256, 64), (2, 64, 1024, 256), (2, 17, 2048, 1024)])
+@pytest.mark.parametrize("B,C,N,M", THREE_NN_CASES)
 def test_nearest_neighbor_interpolate(B, C, N, M):
     F = _F()
-    pts = cloud(9, B, N)
-    ctr = pts[:, :, :M].clone()                            # centres coincide with points: d = 0 -> clamp 1e-10
-    cf = gen(10, B, C, M)
+    pts, ctr, cf = three_nn_inputs(B, C, N, M)
     out = F.nearest_neighbor_interpolate(pts.cuda(), ctr.cuda(), cf.cuda())
     out_o = P.nearest_neighbor_interpolate(pts, ctr, cf)
     assert_close(out, out_o, 2e-6, "3-NN interpolate")
-    ref = _ref()
-    o, idx, w = ref.three_nearest_neighbors_interpolate_forward(pts.cuda(), ctr.cuda(), cf.cuda())
+    k = key("three_nn", B, C, N, M)
     idx_o, w_o = P.three_nn(pts, ctr)
-    assert torch.equal(idx.cpu(), idx_o), "3-NN indices: oracle vs reference kernel"
-    assert_close(out, o, 1e-6, "3-NN interpolate vs reference kernel")
+    REF.exact(k + "/idx", idx_o, "3-NN indices: oracle vs reference kernel")
+    REF.close(k + "/out", out, 1e-6, "3-NN interpolate vs reference kernel")
 
 
 def test_gather():
@@ -181,10 +207,7 @@ def test_fused_path_voxel_indices_bit_exact_b32():
     lion_voxel_coords against the reference's own kernel fed with torch-CUDA indices."""
     F = _F()
     B, N, r = 32, 2048, 32
-    coords = cloud(29, B, N, spread=0.41)
-    feats = gen(30, B, 8, N)
+    coords, feats = fused_inputs()
     _, vox = F.voxel_coords(coords.cuda(), r)
-    _, vox_t = _voxelization_torch(coords.cuda(), r)
-    o, ind, cnt = _ref().avg_voxelize_forward(feats.cuda(), vox_t.contiguous(), r)
     out = F.avg_voxelize(feats.cuda(), vox, r)
-    assert_close(out.view(B, 8, -1), o, 1e-5, "avg_voxelize at B=32 on torch-CUDA voxel indices")
+    REF.close("fused_b32/out", out.view(B, 8, -1), 1e-5, "avg_voxelize at B=32 on torch-CUDA voxel indices")
